@@ -456,6 +456,20 @@ class Leg:
         inp_sel = np.ascontiguousarray(self.h_in.numpy()[:, :, sel])
         return parity_check(self.w, sel, self.steps_done, self.T, inp_sel, rows, st)
 
+    def dump_outputs(self, path, steps, n_rows=2048, max_bytes=60 << 20):
+        """Write what the last step returned to its caller: the output rows of a fixed, seeded sample of voices
+        (out_rows.npy [T][n][64], their indices in out_rows_voices.npy) and the mix bus (mix.npy [T][64]).
+        The sample shrinks for long steps so that the rows stay under `max_bytes` (the whole dump under 64 MB).
+        Must run before anything else launches the graph again."""
+        os.makedirs(path, exist_ok=True)
+        n = max(1, min(n_rows, self.V, max_bytes // (self.T * BLOCK * 4)))
+        sel = np.sort(np.random.default_rng(0).choice(self.V, n, replace=False))
+        idx = self.torch.from_numpy(sel).to(self.d_out.device)
+        np.save(os.path.join(path, "out_rows.npy"), self.d_out[:, 0].index_select(1, idx).cpu().numpy())
+        np.save(os.path.join(path, "out_rows_voices.npy"), sel.astype(np.float64))
+        if self.use_mix:
+            np.save(os.path.join(path, "mix.npy"), self.d_mix[(steps - 1) & 1][:, 0].cpu().numpy())  # as step() picks it
+
     def detach_collective(self):
         """Local mix only from here on (used to measure what the collective costs)."""
         if self.peer is not None:
@@ -516,6 +530,8 @@ def run_cuda_arm(args):
 
     sampler = ClockSampler(physical_gpu_index(local_rank)) if rank == 0 else None
     ms, launches = leg.timed(args.steps, args.warmup, sampler)
+    if args.dump_outputs and rank == 0:
+        leg.dump_outputs(args.dump_outputs, args.steps)
     vs_per_step = leg.V * T * BLOCK
     vs_job = (V if strong else V * world) * T * BLOCK
     value = vs_job * args.steps / (ms * 1e-3)
@@ -748,7 +764,12 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the contract S / M e2e legs")
     ap.add_argument("--no-parity", action="store_true", help="skip the bit-comparison with the CPU checker")
     ap.add_argument("--no-other-scaling", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (a seeded sample of up to 2048 voice "
+                         "rows, at most 64 MB in all, and the mix bus) to DIR as .npy files")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_cuda_arm(args)

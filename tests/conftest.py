@@ -22,14 +22,14 @@ def port():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The compiled reference itself; only present where oracle/_ref was built."""
-    from oracle import bindings
-    if not bindings.ref_available():
-        if os.path.isdir("/root/reference/source/DSP"):
-            bindings.build("ref")
-        else:
-            pytest.skip("oracle/_ref/libmlref.so not built (no /root/reference here)")
-    return bindings.RefOracle()
+    """The compiled reference itself, as recorded in tests/golden/reference.npz (tests/recorded_reference.py)."""
+    from tests import recorded_reference
+    return recorded_reference.oracle()
+
+
+def pytest_sessionfinish(session):
+    from tests import recorded_reference
+    recorded_reference.save()
 
 
 @pytest.fixture(scope="session")

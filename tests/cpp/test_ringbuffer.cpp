@@ -1,16 +1,24 @@
 // tests/cpp/test_ringbuffer.cpp -- CPU-only.  mlb::DSPBuffer and mlb::BatchedSignalProcessBuffer
 // (include/mlb200_host.hpp) must behave like the reference's ml::DSPBuffer / ml::SignalProcessBuffer.
-// With -DHAVE_REFERENCE (only where /root/reference exists) the ring is driven in lockstep with the
-// reference's own class on random operation sequences, and the batched process buffer against a
-// restatement of the reference's per-vector loop (MLSignalProcessBuffer.cpp:57-78) built from the
-// reference's DSPBuffer.  Without it, self-consistency checks only.  Mirrors Tests/dspBufferTest.cpp.
+// The ring is driven on random operation sequences, and the batched process buffer is compared with a
+// restatement of the reference's per-vector loop (MLSignalProcessBuffer.cpp:57-78) built from the reference's
+// DSPBuffer.  Everything read back is hashed per run (tests/cpp/lockstep_digest.h): built with -DHAVE_REFERENCE
+// (the reference sources on the include path) the reference's classes also run in lockstep and `record` writes
+// their hashes; built without, our hashes must equal the recorded ones.  Mirrors Tests/dspBufferTest.cpp.
+//   test_ringbuffer <digest file> [record]
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
+#include <string>
 #include <vector>
 
 #include "mlb200_host.hpp"
+#include "lockstep_digest.h"
 #ifdef HAVE_REFERENCE
 #include "MLDSPBuffer.h"
+#define REF(...) __VA_ARGS__
+#else
+#define REF(...) (void)0
 #endif
 
 static int g_fail = 0, g_checks = 0;
@@ -18,8 +26,10 @@ static int g_fail = 0, g_checks = 0;
 
 static unsigned rnd(unsigned& s) { s = s * 1664525u + 1013904223u; return s >> 8; }
 
-int main()
+int main(int argc, char** argv)
 {
+  if (argc < 2) { std::printf("usage: test_ringbuffer <digest file> [record]\n"); return 2; }
+  Digests d(argv[1], argc > 2 && std::strcmp(argv[2], "record") == 0, HAVE_REFERENCE_SOURCES);
   // ---- basic semantics (Tests/dspBufferTest.cpp: sizes, wrap, overflow) ----
   {
     mlb::DSPBuffer b;
@@ -38,15 +48,17 @@ int main()
     float v[64];
     REQUIRE(!b.readVector(v) && v[0] == 0.f);  // silence, nothing consumed
   }
-#ifdef HAVE_REFERENCE
   // ---- lockstep with the reference's DSPBuffer on random operation sequences ----
   for (unsigned seed = 1; seed <= 20; ++seed)
   {
     unsigned s = seed;
-    ml::DSPBuffer ref;
+    REF(ml::DSPBuffer ref);
     mlb::DSPBuffer mine;
+    Hash hr, hm;
     const int size = 64 + (int)(rnd(s) % 900);
-    REQUIRE(ref.resize(size) == mine.resize(size));
+    const size_t cap = mine.resize(size);
+    REF(REQUIRE(ref.resize(size) == cap); hr.add((uint64_t)cap));
+    hm.add((uint64_t)cap);
     std::vector<float> src(4096), a(4096), b(4096);
     float counter = 0;
     for (int step = 0; step < 400; ++step)
@@ -56,39 +68,47 @@ int main()
       if (op <= 1)
       {
         for (size_t i = 0; i < n; ++i) src[i] = counter++;
-        ref.write(src.data(), n);
+        REF(ref.write(src.data(), n));
         mine.write(src.data(), n);
       }
       else if (op == 2)
       {
-        const size_t ra = ref.read(a.data(), n), rb = mine.read(b.data(), n);
-        REQUIRE(ra == rb);
-        for (size_t i = 0; i < ra; ++i) REQUIRE(a[i] == b[i]);
+        const size_t rb = mine.read(b.data(), n);
+        REF(const size_t ra = ref.read(a.data(), n); REQUIRE(ra == rb);
+            for (size_t i = 0; i < ra; ++i) REQUIRE(a[i] == b[i]);
+            hr.add((uint64_t)ra), hr.add(a.data(), ra * sizeof(float)));
+        hm.add((uint64_t)rb), hm.add(b.data(), rb * sizeof(float));
       }
       else if (op == 3)
       {
-        ml::DSPVector rv = ref.read();
         float mv[64];
         mine.readVector(mv);
-        for (int i = 0; i < 64; ++i) REQUIRE(rv[i] == mv[i]);
+        REF(ml::DSPVector rv = ref.read(); for (int i = 0; i < 64; ++i) REQUIRE(rv[i] == mv[i]);
+            hr.add(rv.getConstBuffer(), 64 * sizeof(float)));
+        hm.add(mv, sizeof mv);
       }
       else
       {
-        ref.discard(n);
+        REF(ref.discard(n));
         mine.discard(n);
       }
-      REQUIRE(ref.getReadAvailable() == mine.getReadAvailable());
+      REF(REQUIRE(ref.getReadAvailable() == mine.getReadAvailable()); hr.add((uint64_t)ref.getReadAvailable()));
+      hm.add((uint64_t)mine.getReadAvailable());
     }
+    REQUIRE(d.check("ring/seed" + std::to_string(seed), hr, hm));
   }
   // ---- overlap-add writer / overlapping reader in lockstep (MLDSPBuffer.h:288-340): windowed frames of
   // `win` samples hopped by win - overlap, as an STFT resynthesis would use them ----
   for (unsigned seed = 1; seed <= 12; ++seed)
   {
     unsigned s = seed * 7919u;
-    ml::DSPBuffer ref;
+    REF(ml::DSPBuffer ref);
     mlb::DSPBuffer mine;
+    Hash hr, hm;
     const int size = 256 + (int)(rnd(s) % 2000);
-    REQUIRE(ref.resize(size) == mine.resize(size));
+    const size_t cap = mine.resize(size);
+    REF(REQUIRE(ref.resize(size) == cap); hr.add((uint64_t)cap));
+    hm.add((uint64_t)cap);
     const size_t win = 16 + rnd(s) % 100, overlap = rnd(s) % win;
     std::vector<float> frame(win), a(4096), b(4096);
     float counter = 1.f;
@@ -98,7 +118,7 @@ int main()
       if (op <= 1)
       {
         for (size_t i = 0; i < win; ++i) frame[i] = (counter += 0.5f);
-        ref.writeWithOverlapAdd(frame.data(), win, overlap);
+        REF(ref.writeWithOverlapAdd(frame.data(), win, overlap));
         mine.writeWithOverlapAdd(frame.data(), win, overlap);
       }
       else
@@ -108,22 +128,25 @@ int main()
         {
           std::fill(a.begin(), a.begin() + win, -1.f);
           std::fill(b.begin(), b.begin() + win, -1.f);
-          ref.readWithOverlap(a.data(), win, overlap);
           mine.readWithOverlap(b.data(), win, overlap);
-          for (size_t i = 0; i < win; ++i) REQUIRE(a[i] == b[i]);
+          REF(ref.readWithOverlap(a.data(), win, overlap); for (size_t i = 0; i < win; ++i) REQUIRE(a[i] == b[i]);
+              hr.add(a.data(), win * sizeof(float)));
+          hm.add(b.data(), win * sizeof(float));
         }
       }
-      REQUIRE(ref.getReadAvailable() == mine.getReadAvailable());
-      REQUIRE(ref.getWriteAvailable() == mine.getWriteAvailable());
+      REF(REQUIRE(ref.getReadAvailable() == mine.getReadAvailable());
+          REQUIRE(ref.getWriteAvailable() == mine.getWriteAvailable());
+          hr.add((uint64_t)ref.getReadAvailable()), hr.add((uint64_t)ref.getWriteAvailable()));
+      hm.add((uint64_t)mine.getReadAvailable()), hm.add((uint64_t)mine.getWriteAvailable());
     }
+    REQUIRE(d.check("overlap/seed" + std::to_string(seed), hr, hm));
   }
   // ---- batched process buffer vs the reference's per-vector loop ----
   {
     const int maxFrames = 1024;
     mlb::BatchedSignalProcessBuffer batched(1, 2, maxFrames);
-    ml::DSPBuffer rin, rout[2];
-    rin.resize(maxFrames);
-    rout[0].resize(maxFrames), rout[1].resize(maxFrames);
+    REF(ml::DSPBuffer rin, rout[2]; rin.resize(maxFrames); rout[0].resize(maxFrames), rout[1].resize(maxFrames));
+    Hash hr, hm;
     float acc_ref = 0.f, acc_mine = 0.f;  // a stateful "processor": running sum + input
     unsigned s = 99;
     std::vector<float> xin(maxFrames), o0(maxFrames), o1(maxFrames), r0(maxFrames), r1(maxFrames);
@@ -133,14 +156,15 @@ int main()
       const int frames = 1 + (int)(rnd(s) % maxFrames);
       for (int i = 0; i < frames; ++i) xin[i] = (t += 0.25f);
       // reference loop (MLSignalProcessBuffer.cpp:47-86)
-      rin.write(xin.data(), frames);
-      while ((int)rout[0].getReadAvailable() < frames)
-      {
-        ml::DSPVector in = rin.read(), a, b;
-        for (int i = 0; i < 64; ++i) { acc_ref += 1.f; a[i] = acc_ref + in[i]; b[i] = -in[i]; }
-        rout[0].write(a), rout[1].write(b);
-      }
-      rout[0].read(r0.data(), frames), rout[1].read(r1.data(), frames);
+      REF(rin.write(xin.data(), frames);
+          while ((int)rout[0].getReadAvailable() < frames)
+          {
+            ml::DSPVector in = rin.read(), a, b;
+            for (int i = 0; i < 64; ++i) { acc_ref += 1.f; a[i] = acc_ref + in[i]; b[i] = -in[i]; }
+            rout[0].write(a), rout[1].write(b);
+          }
+          rout[0].read(r0.data(), frames), rout[1].read(r1.data(), frames);
+          hr.add(r0.data(), frames * sizeof(float)), hr.add(r1.data(), frames * sizeof(float)));
       // batched
       const float* ins[1] = {xin.data()};
       float* outs[2] = {o0.data(), o1.data()};
@@ -153,11 +177,15 @@ int main()
             out[(v * 2 + 1) * 64 + i] = -in[v * 64 + i];
           }
       });
-      for (int i = 0; i < frames; ++i) { REQUIRE(o0[i] == r0[i]); REQUIRE(o1[i] == r1[i]); }
+      REF(for (int i = 0; i < frames; ++i) { REQUIRE(o0[i] == r0[i]); REQUIRE(o1[i] == r1[i]); });
+      hm.add(o0.data(), frames * sizeof(float)), hm.add(o1.data(), frames * sizeof(float));
     }
+    REQUIRE(d.check("process_buffer", hr, hm));
+    (void)acc_ref;
   }
-  std::printf("(checked against the reference's DSPBuffer)\n");
-#endif
+  if (!d.finish()) ++g_fail;
+  std::printf("(checked %s)\n", HAVE_REFERENCE_SOURCES ? "in lockstep with the reference's DSPBuffer"
+                                                        : "against the reference's recorded digests");
   std::printf("%s: %d checks, %d failed\n", g_fail ? "FAILED" : "ALL PASSED", g_checks, g_fail);
   return g_fail ? 1 : 0;
 }

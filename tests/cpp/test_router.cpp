@@ -4,19 +4,33 @@
 // all-notes-off; polyphonic and unison) goes (a) into ml::EventsToSignals and (b) through the router
 // into per-voice event records and then through a Voice bank -- the C port on the CPU, or the CUDA bank
 // when run with the argument "gpu".  All 8 rows of every voice must agree bit for bit.
+//
+// Built with -DHAVE_REFERENCE (linked with libmle2s.so) the reference runs beside ours and `record` writes the
+// hash of its rows per phrase (tests/cpp/lockstep_digest.h); built without, our rows must have the recorded hash.
+//   test_router <digest file> [gpu] [record]
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 #include <vector>
 
 #include "mlb200_events.hpp"
+#include "lockstep_digest.h"
+
+#ifdef HAVE_REFERENCE
+#define REF(...) __VA_ARGS__
+#else
+#define REF(...) (void)0
+#endif
 
 extern "C" {
+#ifdef HAVE_REFERENCE
 struct mle2s_full;
 mle2s_full* mle2s_full_create(float sr, int polyphony, float glideSeconds, float driftAmount, int unison, int mpe);
 void mle2s_full_destroy(mle2s_full*);
 void mle2s_full_add_event(mle2s_full*, int type, int channel, int sourceIdx, int time, float v1, float v2);
 void mle2s_full_process(mle2s_full*, int start, float* out);
+#endif
 struct mlport_voice_bank;
 mlport_voice_bank* mlport_bank_create(int V, float sr, const int32_t* voiceIndex, const float* glideSeconds,
                                       const float* driftAmount, const float* pitchBend, unsigned flags);
@@ -110,19 +124,19 @@ static std::vector<mlb::Event> make_phrase(int T, int seed)
   return ev;
 }
 
-static int run_case(int polyphony, bool unison, int seed, bool gpu, bool mpe = false)
+static int run_case(Digests& d, int polyphony, bool unison, int seed, bool gpu, bool mpe = false)
 {
   const int T = 400, P = polyphony;
   const float sr = 48000.f, glide = 0.03f, drift = 0.5f;
   const auto phrase = mpe ? make_mpe_phrase(T, seed) : make_phrase(T, seed);
 
-  mle2s_full* ref = mle2s_full_create(sr, P, glide, drift, unison ? 1 : 0, mpe ? 1 : 0);
+  REF(mle2s_full* ref = mle2s_full_create(sr, P, glide, drift, unison ? 1 : 0, mpe ? 1 : 0));
   mlb::VoiceRouter router(P, mpe ? mlb::VoiceRouter::kMPE : mlb::VoiceRouter::kMIDI);
   const int NR = router.recordCount(), first = mpe ? 1 : 0;  // bank voices; index of the first channel voice
   router.setUnison(unison);
   for (const auto& e : phrase)
   {
-    mle2s_full_add_event(ref, e.type, e.channel, e.sourceIdx, e.time, e.value1, e.value2);
+    REF(mle2s_full_add_event(ref, e.type, e.channel, e.sourceIdx, e.time, e.value1, e.value2));
     router.addEvent(e);
   }
   std::vector<float> want((size_t)T * P * 8 * 64);
@@ -130,10 +144,10 @@ static int run_case(int polyphony, bool unison, int seed, bool gpu, bool mpe = f
   int overflow = 0;
   for (int t = 0; t < T; ++t)
   {
-    mle2s_full_process(ref, t * 64, want.data() + (size_t)t * P * 8 * 64);  // [P][8][64]
+    REF(mle2s_full_process(ref, t * 64, want.data() + (size_t)t * P * 8 * 64));  // [P][8][64]
     overflow += router.processVector(t * 64, recs.data() + (size_t)t * NR);
   }
-  mle2s_full_destroy(ref);
+  REF(mle2s_full_destroy(ref));
   if (overflow) { std::printf("  (phrase needs > %d note events per voice-vector %d times)\n", MLB_VOICE_MAX_EVENTS, overflow); return 1; }
 
   // bank voice b is reference voice b + (mpe ? 0 : 1); MPE: voice 0 = the main voice, MIDI bend range 7, the channel
@@ -167,47 +181,60 @@ static int run_case(int polyphony, bool unison, int seed, bool gpu, bool mpe = f
     mlport_bank_process(b, T, recs.data(), got.data(), 1);
     mlport_bank_destroy(b);
   }
-  size_t bad = 0, total = 0;
+  size_t bad = 0, total = 0;  // word comparisons, with the reference beside ours
   double energy = 0;
+  std::vector<float> ours(want.size());  // [T][P][8][64], the reference's layout
   for (int t = 0; t < T; ++t)
     for (int v = 0; v < P; ++v)
       for (int r = 0; r < 8; ++r)
         for (int n = 0; n < 64; ++n)
         {
-          const float a = want[(((size_t)t * P + v) * 8 + r) * 64 + n];
           const float b = got[(((size_t)t * 8 + r) * NR + v + first) * 64 + n];
-          uint32_t ua, ub;
-          std::memcpy(&ua, &a, 4), std::memcpy(&ub, &b, 4);
-          if (ua != ub)
-          {
-            if (bad < 5) std::printf("  mismatch t=%d voice=%d row=%d n=%d: reference %g (%08x) ours %g (%08x)\n", t, v, r, n, a, ua, b, ub);
-            ++bad;
-          }
+          ours[(((size_t)t * P + v) * 8 + r) * 64 + n] = b;
+          REF(const float a = want[(((size_t)t * P + v) * 8 + r) * 64 + n];
+              uint32_t ua, ub;
+              std::memcpy(&ua, &a, 4), std::memcpy(&ub, &b, 4);
+              if (ua != ub)
+              {
+                if (bad < 5) std::printf("  mismatch t=%d voice=%d row=%d n=%d: reference %g (%08x) ours %g (%08x)\n", t, v, r, n, a, ua, b, ub);
+                ++bad;
+              });
           ++total;
-          if (r == 1) energy += a;
+          if (r == 1) energy += b;
         }
-  std::printf("  %s polyphony %d %s seed %d: %zu of %zu words differ (gate sum %.1f, %zu events)\n", mpe ? "MPE " : "MIDI", P,
-              unison ? "unison" : "poly", seed, bad, total, energy, phrase.size());
-  return bad ? 1 : (energy > 10 ? 0 : 1);
+  Hash hr, hm;
+  REF(hr.add(want.data(), want.size() * sizeof(float)));
+  hm.add(ours.data(), ours.size() * sizeof(float));
+  const std::string name = std::string(mpe ? "mpe" : "midi") + "/P" + std::to_string(P) + (unison ? "/unison" : "/poly") +
+                           "/seed" + std::to_string(seed);
+  const bool recorded = d.check(name, hr, hm);
+  std::printf("  %s polyphony %d %s seed %d: ", mpe ? "MPE " : "MIDI", P, unison ? "unison" : "poly", seed);
+  REF(std::printf("%zu of %zu words differ from the reference, ", bad, total));
+  std::printf("digest %s the reference's (gate sum %.1f, %zu events)\n", recorded ? "equals" : "DIFFERS FROM", energy,
+              phrase.size());
+  return (bad || !recorded) ? 1 : (energy > 10 ? 0 : 1);
 }
 
 int main(int argc, char** argv)
 {
-  const bool gpu = argc > 1 && std::strcmp(argv[1], "gpu") == 0;
+  if (argc < 2) { std::printf("usage: test_router <digest file> [gpu] [record]\n"); return 2; }
+  bool gpu = false, record = false;
+  for (int i = 2; i < argc; ++i) gpu |= std::strcmp(argv[i], "gpu") == 0, record |= std::strcmp(argv[i], "record") == 0;
+  Digests d(argv[1], record, HAVE_REFERENCE_SOURCES);
   if (gpu && mlb_init(0) != MLB_OK)
   {
     std::printf("no device: %s\n", mlb_last_error());
     return 77;
   }
   int fails = 0;
-  fails += run_case(4, false, 1, gpu);
-  fails += run_case(8, false, 2, gpu);
-  fails += run_case(2, false, 3, gpu);
-  fails += run_case(4, true, 4, gpu);
-  fails += run_case(16, false, 5, gpu);
-  fails += run_case(8, false, 6, gpu, true);
-  fails += run_case(4, false, 7, gpu, true);
-  fails += run_case(15, false, 8, gpu, true);
+  fails += run_case(d, 4, false, 1, gpu);
+  fails += run_case(d, 8, false, 2, gpu);
+  fails += run_case(d, 2, false, 3, gpu);
+  fails += run_case(d, 4, true, 4, gpu);
+  fails += run_case(d, 16, false, 5, gpu);
+  fails += run_case(d, 8, false, 6, gpu, true);
+  fails += run_case(d, 4, false, 7, gpu, true);
+  fails += run_case(d, 15, false, 8, gpu, true);
   // ---- limits are reported, not hidden ----
   {
     mlb::VoiceRouter router(1);  // one voice: every note steals it
@@ -227,6 +254,7 @@ int main(int argc, char** argv)
     std::printf("  overflow and unsupported-event reporting: %s\n", ok ? "ok" : "WRONG");
     fails += ok ? 0 : 1;
   }
+  if (!d.finish()) ++fails;
   std::printf(fails ? "FAILED\n" : "ALL PASSED\n");
   return fails ? 1 : 0;
 }

@@ -11,17 +11,12 @@ pytestmark = pytest.mark.gpu
 EXACT_CASES = [c for c in wl.SWEPT_CASES if c != "lopass_mod"]
 
 
-def _checker(port):
-    from oracle import bindings
-    return bindings.RefOracle() if bindings.ref_available() else port
-
-
 @pytest.mark.parametrize("name", EXACT_CASES)
 @pytest.mark.parametrize("n_voices,n_blocks,splits", [(37, 7, (3, 4)), (200, 5, None)])
-def test_swept_filters_bit_exact(gpu, port, name, n_voices, n_blocks, splits):
+def test_swept_filters_bit_exact(gpu, port, ref, name, n_voices, n_blocks, splits):
     w = wl.swept_filter_case(name, n_voices, n_blocks)
     inp = w.inputs(n_blocks)
-    ro, _, rs = _checker(port).run(w.spec, n_voices, n_blocks, inp, w.state, w.coef)
+    ro, _, rs = ref.run(w.spec, n_voices, n_blocks, inp, w.state, w.coef)
     _, pm, _ = port.run(w.spec, n_voices, n_blocks, inp, w.state, w.coef, want_mix=True, mix_mode=1)
     fused_expected = name in ("lopass_v", "sine_lopass_v_gain")
     for flags in ((0, gpu.FLAG_FORCE_GENERIC) if fused_expected else (0,)):
@@ -49,13 +44,13 @@ def test_lopass_v_equals_the_reference_operator_itself(gpu, ref):
     assert_same_bits(go[:, 0, 0], want, "LOPASS_V vs Lopass::operator()(vx, omega, k)")
 
 
-def test_fused_swept_chain_large_bank_default_launch_shape(gpu, port):
+def test_fused_swept_chain_large_bank_default_launch_shape(gpu, port, ref):
     """SineGen -> Lopass(coefficient rows) -> gain through the persistent multi-plane chain grid
     (20 000 voices > 4 * SMs groups: dynamic work units, state hopping), ragged last group, mix bus."""
     V, T = 20000 + 13, 16
     w = wl.swept_filter_case("sine_lopass_v_gain", V, T)
     inp = w.inputs(T)
-    ro, _, rs = _checker(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=16)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=16)
     _, pm, _ = port.run(w.spec, V, T, inp, w.state, w.coef, want_out=False, want_mix=True, mix_mode=1, nthreads=16)
     go, gm, gs, kname = run_gpu(gpu, w, T, inp, want_mix=True, splits=(9, 7))
     assert kname.startswith("fused:"), kname
@@ -64,14 +59,14 @@ def test_fused_swept_chain_large_bank_default_launch_shape(gpu, port):
     assert_state_equal(gs, rs, "swept chain state")
 
 
-def test_lopass_mod_device_coefficients_within_tolerance(gpu, port):
+def test_lopass_mod_device_coefficients_within_tolerance(gpu, port, ref):
     """LOPASS_MOD designs the coefficients on the device (CUDA sinf, not glibc's): the approximate
     variant.  Stated tolerance (DESIGN.md 5): 2e-5 of the output's peak over 12 blocks of sweeps
     with k >= 0.05 (Q <= 20)."""
     V, T = 150, 12
     w = wl.swept_filter_case("lopass_mod", V, T)
     inp = w.inputs(T)
-    ro, _, _ = _checker(port).run(w.spec, V, T, inp, w.state, w.coef)
+    ro, _, _ = ref.run(w.spec, V, T, inp, w.state, w.coef)
     go, _, _, kname = run_gpu(gpu, w, T, inp)
     err = float(np.abs(go - ro).max() / np.abs(ro).max())
     print("LOPASS_MOD max error relative to peak:", err, kname)

@@ -4,10 +4,9 @@ The small-size tests in test_gpu_chain.py cover the edge cases; these cover the 
 tools/bench_configs.py actually time: the persistent 12-warp x 148-CTA chain grid with (group, chunk)
 work units and state hopping between warps (only taken above 4 * SMs voice groups), the 16-slice
 three-stream host pipeline behind the e2e number, the FDN kernel at 16 384 voices and the graph
-interpreter's stage pipeline at 1 024 x 256 nodes.  The checker is the reference itself compiled in
-place (oracle/_ref, all host threads) for rows and state, and the port for the mix bus in the device
-summation order; where oracle/_ref was not built the port (pinned to it bit-for-bit by
-test_oracle_port_vs_ref.py) stands in.
+interpreter's stage pipeline at 1 024 x 256 nodes.  The checker is the reference itself for rows and state
+(as recorded in tests/golden/reference.npz: the port's rows must have the reference's digest), and the port
+for the mix bus in the device summation order.
 """
 import os
 
@@ -20,12 +19,6 @@ from tests.common import assert_same_bits, assert_state_equal
 pytestmark = pytest.mark.gpu
 
 NTHREADS = max(1, len(os.sched_getaffinity(0)))
-
-
-def _oracle(port):
-    """The compiled reference where it exists, else the port."""
-    from oracle import bindings
-    return bindings.RefOracle() if bindings.ref_available() else port
 
 
 def _device_run(gpu, w, T, inp, want_mix=False, flags=0):
@@ -51,12 +44,12 @@ def _device_run(gpu, w, T, inp, want_mix=False, flags=0):
     return out, mix, st, name
 
 
-def test_config_a_full_size_device_path(gpu, port):
+def test_config_a_full_size_device_path(gpu, port, ref):
     """Config A, 65 536 voices x 64 blocks, default launch shape (W=12 x 148 CTAs, 6 time chunks)."""
     V, T = 65536, 64
     w = wl.config_a(V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     _, pm, _ = port.run(w.spec, V, T, inp, w.state, w.coef, want_out=False, want_mix=True, mix_mode=1,
                         nthreads=NTHREADS)
     go, gm, gs, name = _device_run(gpu, w, T, inp, want_mix=True)
@@ -70,14 +63,14 @@ def test_config_a_full_size_device_path(gpu, port):
     assert np.abs(gm - ref_mix).max() <= tol
 
 
-def test_config_a_full_size_host_pipeline(gpu, port, monkeypatch):
+def test_config_a_full_size_host_pipeline(gpu, port, ref, monkeypatch):
     """The same bank through mlb_graph_process_host: 16 voice slices, H2D / kernel / D2H on three
     streams -- the path behind bench.py's e2e number.  Two successive calls (progress words carry)."""
     monkeypatch.delenv("MLB_HOST_SLICES", raising=False)
     V, T = 65536, 64
     w = wl.config_a(V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     _, pm, _ = port.run(w.spec, V, T, inp, w.state, w.coef, want_out=False, want_mix=True, mix_mode=1,
                         nthreads=NTHREADS)
     g = gpu.VoiceGraph(w.spec, V)
@@ -97,11 +90,11 @@ def test_config_a_full_size_host_pipeline(gpu, port, monkeypatch):
     assert_state_equal(gs, rs, "config A host pipeline state")
 
 
-def test_config_3_full_size(gpu, port):
+def test_config_3_full_size(gpu, port, ref):
     V, T = 65536, 64
     w = wl.config_3(V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     go, _, gs, name = _device_run(gpu, w, T, inp)
     assert name.startswith("fused:"), name
     assert_same_bits(go, ro, "config 3 65536x64 out")
@@ -109,23 +102,23 @@ def test_config_3_full_size(gpu, port):
 
 
 @pytest.mark.parametrize("kind", ["lopass", "bell"])
-def test_config_2_full_size(gpu, port, kind):
+def test_config_2_full_size(gpu, port, ref, kind):
     V, T = 4096, 64
     w = wl.config_2(kind, V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     go, _, gs, name = _device_run(gpu, w, T, inp)
     assert name.startswith("fused:"), name
     assert_same_bits(go, ro, "config 2 out " + kind)
     assert_state_equal(gs, rs, "config 2 state " + kind)
 
 
-def test_config_4_full_size(gpu, port):
+def test_config_4_full_size(gpu, port, ref):
     """16 384 voices x 16 blocks of 3-op FM -> FDN<8>, in two launches (ring write index carries)."""
     V, T = 16384, 16
     w = wl.config_4(V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     _, pm, _ = port.run(w.spec, V, T, inp, w.state, w.coef, want_out=False, want_mix=True, mix_mode=1,
                         nthreads=NTHREADS)
     go, gm, gs, name = _device_run(gpu, w, T, inp, want_mix=True)
@@ -136,23 +129,23 @@ def test_config_4_full_size(gpu, port):
     assert np.abs(go).max() > 0.1
 
 
-def test_config_5_full_size(gpu, port):
+def test_config_5_full_size(gpu, port, ref):
     """1 024 instances x 256-node chain x 16 blocks through the interpreter's stage pipeline."""
     V, T = 1024, 16
     w = wl.config_5(V, 256)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, None, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, None, w.state, w.coef, nthreads=NTHREADS)
     go, _, gs, name = _device_run(gpu, w, T, None)
     assert name.startswith("generic"), name
     assert_same_bits(go, ro, "config 5 1024x256x16 out " + name)
     assert_state_equal(gs, rs, "config 5 state")
 
 
-def test_config_6_full_size(gpu, port):
+def test_config_6_full_size(gpu, port, ref):
     """4 096 Aaltoverb reverbs x 16 blocks (SURVEY 8f row 2) at the benchmarked size."""
     V, T = 4096, 16
     w = wl.config_6(V)
     inp = w.inputs(T)
-    ro, _, rs = _oracle(port).run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
+    ro, _, rs = ref.run(w.spec, V, T, inp, w.state, w.coef, nthreads=NTHREADS)
     go, _, gs, name = _device_run(gpu, w, T, inp)
     assert_same_bits(go, ro, "config 6 4096x16 out " + name)
     assert_state_equal(gs, rs, "config 6 state")

@@ -1,4 +1,6 @@
 """Stateless elementwise ops (every DEFINE_OP* of MLDSPOps.h) on the GPU vs the port oracle."""
+import zlib
+
 import numpy as np
 import pytest
 
@@ -30,7 +32,7 @@ def make_inputs(nin, n_rows, seed):
 def test_map_op(gpu, port, name):
     nin = OP_TABLE[name][1]
     n_rows = 37
-    x = make_inputs(nin, n_rows, hash(name) % 1000)
+    x = make_inputs(nin, n_rows, zlib.crc32(name.encode()) % 1000)  # the same inputs in every process
     g = GraphSpec()
     g.output(g.node(name, *[g.input(k) for k in range(nin)]))
     inp = np.ascontiguousarray(x[:, None].transpose(1, 0, 2, 3))  # [T=1][nin][V=n_rows][64]
@@ -38,9 +40,12 @@ def test_map_op(gpu, port, name):
     want = want[0, 0]
     got = gpu.map_host(name, x[0], x[1] if nin > 1 else None, x[2] if nin > 2 else None)
     if name in HW_APPROX:
-        # rcpps/rsqrtps treat denormal operands as zero; the GPU does not: compare normal inputs
+        # rcpps/rsqrtps treat denormal operands as zero, and flush a denormal reciprocal (of |b| > 1 / FLT_MIN) to
+        # zero; the GPU does neither: compare normal inputs
         tiny = np.finfo(np.float32).tiny
         normal = np.all((np.abs(x[:nin]) >= tiny) | (x[:nin] == 0) | ~np.isfinite(x[:nin]), axis=0)
+        if name == "DIVIDE_APPROX":
+            normal &= ~(np.abs(x[1]) > np.float32(1.0) / tiny)
         ok = np.isfinite(want) & np.isfinite(got) & normal
         rel = np.abs(got[ok] - want[ok]) / np.maximum(np.abs(want[ok]), 1e-30)
         assert rel.max() <= 2 * HW_APPROX[name]

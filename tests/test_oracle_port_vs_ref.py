@@ -1,5 +1,5 @@
-"""The plain-C port against the compiled reference on fresh random inputs (only where
-oracle/_ref exists: the authoring container, or a GPU box that received the built .so)."""
+"""The plain-C port against the compiled reference on fresh random inputs (the reference's results as
+recorded in tests/golden/reference.npz, see tests/recorded_reference.py)."""
 import numpy as np
 import pytest
 

@@ -16,9 +16,10 @@ def _signal(T, V, seed):
 @pytest.mark.parametrize("octaves", [1, 2, 3, 4])
 def test_port_equals_reference_resamplers(ref, direction, octaves):
     from oracle.bindings import Resampler
+    from tests import recorded_reference
     V = 9
     x = _signal(37, V, 5 + octaves)
-    a, b = Resampler("ref", direction, octaves, V), Resampler("port", direction, octaves, V)
+    a, b = recorded_reference.resampler(direction, octaves, V), Resampler("port", direction, octaves, V)
     ya = np.concatenate([a.process(x[:10]), a.process(x[10:])])
     yb = np.concatenate([b.process(x[:10]), b.process(x[10:23]), b.process(x[23:])])
     a.close(), b.close()

@@ -285,9 +285,8 @@ def _run_gpu_case(tmp_path, case, V, T, inp):
 @pytest.mark.gpu
 @pytest.mark.parametrize("case,V,T", [("chain", 70, 6), ("sine", 33, 4), ("reverb", 37, 24), ("shelf", 40, 5),
                                       ("kitchen", 35, 20)])
-def test_traced_examples_on_gpu(gpu, port, tmp_path, case, V, T):
-    from oracle import bindings
-    O = bindings.RefOracle() if bindings.ref_available() else port
+def test_traced_examples_on_gpu(gpu, port, ref, tmp_path, case, V, T):
+    O = ref
     g, coef, state = traced(case, V)
     inp = None
     if case == "reverb":
@@ -304,11 +303,10 @@ def test_traced_examples_on_gpu(gpu, port, tmp_path, case, V, T):
         # output 1 is built on Peak / RMS (the CPU's 12-bit rsqrt approximation): tolerance-only off the CPU
         assert_same_bits(got[:, 0], want[:, 0], "kitchen output 0 traced on the GPU")
         assert np.abs(got[:, 1] - want[:, 1]).max() <= 2e-3 * np.abs(want[:, 1]).max()
-        if bindings.ref_available():
-            assert_same_bits(got[:, 0, 7], O.kitchen(inp[:, :, 0])[:, 0], "GPU vs the reference build of kitchen_body.h")
+        assert_same_bits(got[:, 0, 7], O.kitchen(inp[:, :, 0])[:, 0], "GPU vs the reference build of kitchen_body.h")
         return
     assert_same_bits(got, want, case + " traced on the GPU")
-    if case == "reverb" and bindings.ref_available():
+    if case == "reverb":
         body, _ = O.aaltoverb(inp[:, :, 0], 1.0, wl.aaltoverb_feedback(0.5, 0.5), 0.1 * 48000)
         assert_same_bits(got[:, :, 5], body, "GPU vs the reverb example's own body")
 

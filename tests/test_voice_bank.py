@@ -8,6 +8,7 @@ import pytest
 
 from madronalib_b200 import workloads as wl
 from tests.common import assert_same_bits
+from tests.recorded_reference import assert_events_to_signals
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "voices.npz")
 ROWS = ["pitch", "gate", "voice", "z", "x", "y", "mod", "time"]
@@ -21,13 +22,8 @@ def port_bank():
 
 @pytest.fixture(scope="module")
 def ref_bank():
-    from oracle import bindings
-    if not os.path.exists(bindings.E2S_LIB):
-        if os.path.isdir("/root/reference/source/app"):
-            bindings.build("ref")
-        else:
-            pytest.skip("oracle/_ref/libmle2s.so not built (no /root/reference here)")
-    return bindings.ref_voice_bank()
+    from tests import recorded_reference
+    return recorded_reference.voice_bank()
 
 
 @pytest.mark.parametrize("sr,seed,flags", [(48000.0, 3, 0), (44100.0, 4, 1), (1000.0, 5, 1)])
@@ -164,12 +160,10 @@ def test_router_c_abi_plus_port_bank_equals_reference(ref_bank, port_bank, mpe, 
     """The C face of the router (mlb_router_*, host only) -> records -> Voice bank (the C port here) against
     the complete reference EventsToSignals, driven from Python with a seeded phrase."""
     from madronalib_b200 import api
-    from oracle.bindings import RefEventsToSignals
     sr, glide, drift, T, P = 48000.0, 0.02, 0.5, 150, polyphony
     rng = np.random.default_rng(21 + polyphony)
-    ref = RefEventsToSignals(sr, P, glide, drift, unison=unison, mpe=mpe)
     router = api.EventRouter(P, api.EventRouter.MPE if mpe else api.EventRouter.MIDI, unison=unison)
-    held = []
+    held, phrase = [], []
     for t in range(T):
         base = t * 64
         evs = []
@@ -190,15 +184,12 @@ def test_router_c_abi_plus_port_bank_equals_reference(ref_bank, port_bank, mpe, 
         if rng.random() < 0.08:
             evs.append((api.EventRouter.SUSTAIN_PEDAL, 1, 0, base + int(rng.integers(64)), float(rng.integers(2)), 0.0))
         for e in evs:
-            ref.add_event(*e)
+            phrase.append(e)
             router.add_event(*e)
     NR = router.n_records
     recs = np.zeros((T, NR), wl.VOICE_EVENTS_DTYPE)
-    want = np.zeros((T, P, 8, 64), np.float32)
     for t in range(T):
-        want[t] = ref.process_vector(t * 64)
         assert router.process_vector(t * 64, recs[t]) == 0
-    ref.close()
     router.close()
     first = 1 if mpe else 0
     idx = np.arange(NR, dtype=np.int32) + (0 if mpe else 1)
@@ -223,9 +214,23 @@ def test_router_c_abi_plus_port_bank_equals_reference(ref_bank, port_bank, mpe, 
     L.mlport_bank_process(h, T, recs.ctypes.data_as(ctypes.c_void_p), got.ctypes.data_as(ctypes.c_void_p), 1)
     L.mlport_bank_destroy.argtypes = [ctypes.c_void_p]
     L.mlport_bank_destroy(h)
-    got = got[:, :, first:, :].transpose(0, 2, 1, 3)  # -> [T][P][8][64]
-    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
-    assert want[:, :, 1].max() > 0.1  # gates happened
+    got = np.ascontiguousarray(got[:, :, first:, :].transpose(0, 2, 1, 3))  # -> [T][P][8][64]
+    assert_events_to_signals(got, lambda: _reference_events_to_signals(sr, P, glide, drift, unison, mpe, T, phrase),
+                             sr, P, glide, drift, unison, mpe, T, phrase)
+    assert got[:, :, 1].max() > 0.1  # gates happened
+
+
+def _reference_events_to_signals(sr, P, glide, drift, unison, mpe, T, phrase):
+    """The complete reference EventsToSignals on `phrase` -> [T][P][8][64]."""
+    from oracle.bindings import RefEventsToSignals
+    ref = RefEventsToSignals(sr, P, glide, drift, unison=unison, mpe=mpe)
+    for e in phrase:
+        ref.add_event(*e)
+    want = np.zeros((T, P, 8, 64), np.float32)
+    for t in range(T):
+        want[t] = ref.process_vector(t * 64)
+    ref.close()
+    return want
 
 
 # ---- fuzz: random phrases, polyphony 1..16, MIDI / unison / MPE, several sample rates, against the complete
@@ -233,20 +238,18 @@ def test_router_c_abi_plus_port_bank_equals_reference(ref_bank, port_bank, mpe, 
 def _fuzz_imports():
     import ctypes
     from madronalib_b200 import api
-    from oracle.bindings import RefEventsToSignals
-    return ctypes, api, RefEventsToSignals
+    return ctypes, api
 
 
 def _router_fuzz_case(seed, PB):
-    ctypes, api, RefEventsToSignals = _fuzz_imports()
+    ctypes, api = _fuzz_imports()
     rng=np.random.default_rng(seed)
     mpe=bool(rng.integers(2)); unison=bool(rng.integers(2)) and not mpe
     P=int(rng.integers(1,17)); sr=float(rng.choice([44100.0,48000.0,96000.0])); glide=float(rng.choice([0.0,0.01,0.05])); drift=float(rng.choice([0.0,1.0]))
     T=int(rng.integers(40,200))
     dens=float(rng.choice([0.1,0.4,0.9]))
-    ref=RefEventsToSignals(sr,P,glide,drift,unison=unison,mpe=mpe)
     router=api.EventRouter(P, 1 if mpe else 0, unison=unison)
-    held=[]
+    held, phrase=[], []
     E=api.EventRouter
     for t in range(T):
         base=t*64
@@ -265,13 +268,13 @@ def _router_fuzz_case(seed, PB):
             elif kind==6: e=(E.CONTROLLER,chan,int(rng.choice([16,73,74,1,123,128,200])),tm,float(rng.choice([0.0,rng.random()])),0.0)
             elif kind==7: e=(int(rng.choice([E.SUSTAIN_PEDAL,E.NOTE_PRESSURE])),chan,int(rng.integers(30,100)),tm,float(rng.random()),0.0)
             else: continue
-            ref.add_event(*e); router.add_event(*e)
+            phrase.append(e); router.add_event(*e)
     NR=router.n_records
-    recs=np.zeros((T,NR),wl.VOICE_EVENTS_DTYPE); want=np.zeros((T,P,8,64),np.float32)
+    recs=np.zeros((T,NR),wl.VOICE_EVENTS_DTYPE)
     over=0
     for t in range(T):
-        want[t]=ref.process_vector(t*64); over+=router.process_vector(t*64,recs[t])
-    ref.close(); router.close()
+        over+=router.process_vector(t*64,recs[t])
+    router.close()
     if over: return "overflow(%d)"%over
     first=1 if mpe else 0
     idx=np.arange(NR,dtype=np.int32)+(0 if mpe else 1)
@@ -286,9 +289,10 @@ def _router_fuzz_case(seed, PB):
     got=np.zeros((T,8,NR,64),np.float32)
     L.mlport_bank_process(h,T,recs.ctypes.data_as(ctypes.c_void_p),got.ctypes.data_as(ctypes.c_void_p),1)
     L.mlport_bank_destroy.argtypes=[ctypes.c_void_p]; L.mlport_bank_destroy(h)
-    got=got[:,:,first:,:].transpose(0,2,1,3)
-    bad=int((got.view(np.uint32)!=want.view(np.uint32)).sum())
-    return "ok" if bad==0 else "MISMATCH %d (mpe=%s unison=%s P=%d sr=%g)"%(bad,mpe,unison,P,sr)
+    got=np.ascontiguousarray(got[:,:,first:,:].transpose(0,2,1,3))
+    assert_events_to_signals(got, lambda: _reference_events_to_signals(sr, P, glide, drift, unison, mpe, T, phrase),
+                             sr, P, glide, drift, unison, mpe, T, phrase)
+    return "ok"
 
 
 @pytest.mark.parametrize("seed", range(24))

@@ -80,21 +80,19 @@ def test_upsample2x_with_a_stateful_process_function_on_the_device(gpu, ref):
         assert_same_bits(go[:, 0, v, :], o, "Upsample2xFunction with a stateful fn, voice %d" % v)
 
 
-def test_traced_upsample_body_on_gpu(gpu, port, tmp_path):
+def test_traced_upsample_body_on_gpu(gpu, port, ref, tmp_path):
     """tests/cpp/upsample_body.h traced and run on the device == the traced graph on the checker == the reference build
     of the same source."""
-    from oracle import bindings
     from tests.test_trace import _run_gpu_case, traced, upsample_input
     V, T = 36, 18
-    O = bindings.RefOracle() if bindings.ref_available() else port
+    O = ref
     g, coef, state = traced("upsample", V)
     inp = upsample_input(T, V)
     _run_gpu_case(tmp_path, "upsample", V, T, inp)
     got = np.fromfile(str(tmp_path / "out.bin"), np.float32).reshape(T, g.n_out, V, 64)
     want, _, _ = O.run(g, V, T, inp, state, coef)
     assert_same_bits(got, want, "upsample body traced on the GPU")
-    if bindings.ref_available():
-        assert_same_bits(got[:, :, 7], O.upsample_body(inp[:, :, 0]), "GPU vs the reference build of upsample_body.h")
+    assert_same_bits(got[:, :, 7], O.upsample_body(inp[:, :, 0]), "GPU vs the reference build of upsample_body.h")
 
 
 @pytest.mark.parametrize("size", [4, 6, 16])
@@ -113,29 +111,26 @@ def test_fdn_of_any_size_on_the_device(gpu, port, ref, size):
         assert_same_bits(go[:, :, v, :], ref.fdn(size, inp[:, 0, v, :], times[:, v], cutoffs, gains), "vs FDN<%d> itself" % size)
 
 
-def test_traced_fdn_body_on_gpu(gpu, port, tmp_path):
+def test_traced_fdn_body_on_gpu(gpu, port, ref, tmp_path):
     """tests/cpp/fdn_body.h (FDN<4> + FDN<6>) traced and run on the device == the reference build of the same source."""
-    from oracle import bindings
     from tests.test_trace import _run_gpu_case, reverb_input, traced
     V, T = 34, 40
-    O = bindings.RefOracle() if bindings.ref_available() else port
+    O = ref
     g, coef, state = traced("fdn", V)
     inp = reverb_input(T, V)
     _run_gpu_case(tmp_path, "fdn", V, T, inp)
     got = np.fromfile(str(tmp_path / "out.bin"), np.float32).reshape(T, g.n_out, V, 64)
     want, _, _ = O.run(g, V, T, inp, state, coef)
     assert_same_bits(got, want, "fdn body traced on the GPU")
-    if bindings.ref_available():
-        assert_same_bits(got[:, :, 5], O.fdn_body(inp[:, :, 0]), "GPU vs the reference build of fdn_body.h")
+    assert_same_bits(got[:, :, 5], O.fdn_body(inp[:, :, 0]), "GPU vs the reference build of fdn_body.h")
 
 
-def test_traced_rows_body_on_gpu(gpu, port, tmp_path):
+def test_traced_rows_body_on_gpu(gpu, port, ref, tmp_path):
     """tests/cpp/rows_body.h (DSPVectorArray<ROWS> as a value, the row operations, Bank with array arguments) traced and
     run on the device == the reference build of the same source."""
-    from oracle import bindings
     from tests.test_trace import _run_gpu_case, traced
     V, T = 33, 12
-    O = bindings.RefOracle() if bindings.ref_available() else port
+    O = ref
     g, coef, state = traced("rows", V)
     n = np.arange(T * 64).reshape(T, 1, 1, 64)
     inp = np.ascontiguousarray(np.repeat((np.float32(110.0 / 48000.0) * (1.0 + 0.3 * np.sin(n * 0.002))).astype(np.float32),
@@ -144,20 +139,18 @@ def test_traced_rows_body_on_gpu(gpu, port, tmp_path):
     got = np.fromfile(str(tmp_path / "out.bin"), np.float32).reshape(T, g.n_out, V, 64)
     want, _, _ = O.run(g, V, T, inp, state, coef)
     assert_same_bits(got, want, "rows body traced on the GPU")
-    if bindings.ref_available():
-        assert_same_bits(got[:, :, 9], O.rows_body(inp[:, :, 0]), "GPU vs the reference build of rows_body.h")
+    assert_same_bits(got[:, :, 9], O.rows_body(inp[:, :, 0]), "GPU vs the reference build of rows_body.h")
 
 
-def test_traced_oversample_body_on_gpu(gpu, port, tmp_path):
+def test_traced_oversample_body_on_gpu(gpu, port, ref, tmp_path):
     """tests/cpp/oversample_body.h (4x / 2x oversampled loops between an Upsampler and a Downsampler; functors and the
     half-band stages called several times per vector) traced and run on the device == the reference build of the same
     source.  Written after the round's last GPU call (the other tests of this file ran in it): every device path it
     takes is one they take -- an MLB_AGAIN node is an ordinary node with another node's word offsets -- and its plan is
     checked in test_planner.py; the first hardware run of this particular graph is the round-end one."""
-    from oracle import bindings
     from tests.test_trace import _run_gpu_case, traced
     V, T = 35, 14
-    O = bindings.RefOracle() if bindings.ref_available() else port
+    O = ref
     g, coef, state = traced("oversample", V)
     rng = np.random.default_rng(9)
     inp = np.ascontiguousarray(np.repeat((rng.standard_normal((T, 1, 1, 64)) * 0.4).astype(np.float32), V, axis=2))
@@ -165,5 +158,4 @@ def test_traced_oversample_body_on_gpu(gpu, port, tmp_path):
     got = np.fromfile(str(tmp_path / "out.bin"), np.float32).reshape(T, g.n_out, V, 64)
     want, _, _ = O.run(g, V, T, inp, state, coef)
     assert_same_bits(got, want, "oversample body traced on the GPU")
-    if bindings.ref_available():
-        assert_same_bits(got[:, :, 11], O.oversample_body(inp[:, :, 0]), "GPU vs the reference build of oversample_body.h")
+    assert_same_bits(got[:, :, 11], O.oversample_body(inp[:, :, 0]), "GPU vs the reference build of oversample_body.h")
